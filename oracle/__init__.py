@@ -4,7 +4,7 @@ May be imported only from tests/, __graft_entry__.smoke() / build() and bench.py
 --impl reference legs.  Never from opentransformer_b200 (the product).
 
 Pinning: (1) committed fixtures produced by the real reference (tests/golden/, tests/test_oracle_golden.py);
-(2) oracle/_ref/ -- the reference's own Python modules byte-compiled by oracle/build_ref.py where /root/reference
-exists (git-ignored, travels with gpurun): tests/test_oracle_ref.py runs the port against the live reference code, and
+(2) oracle/_ref/ -- the reference's own Python modules byte-compiled by oracle/build_ref.py (git-ignored):
+tests/golden/make_reference_checks.py records from it what the reference computes for tests/test_oracle_ref.py, and
 bench.py's reference arm times the reference itself (cpu_baseline.kind "reference"; "port" only when _ref is absent).
 """

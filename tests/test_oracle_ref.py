@@ -1,21 +1,19 @@
-"""The oracle port against the REFERENCE ITSELF, where oracle/_ref exists (the reference's own Python modules, byte-compiled
-by oracle/build_ref.py in the build container; git-ignored, travels with gpurun).  Complements tests/test_oracle_golden.py
-(committed fixtures): here the reference code runs live on fresh random models.  Nothing reads /root/reference."""
+"""The oracle port against the reference's own modules on fresh random models: encoder states, the whole recognize() and the
+training loss / gradients.  Weights and inputs are drawn from seeds here; what the reference computed for them is stored in
+tests/golden/reference_checks.pt (tests/golden/make_reference_checks.py runs the reference on exactly these cases).
+Complements tests/test_oracle_golden.py, whose fixtures pin the reference's configurations with its own initialisation."""
+import math
 import os
-import sys
 
 import pytest
 import torch
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-if ROOT not in sys.path:
-    sys.path.insert(0, ROOT)
+from oracle import beam_search as obs
+from oracle import speech_model as om
 
-from oracle import beam_search as obs      # noqa: E402
-from oracle import build_ref               # noqa: E402
-from oracle import speech_model as om      # noqa: E402
-
-pytestmark = pytest.mark.skipif(build_ref.load() is None, reason='oracle/_ref not built (no reference tree in this environment)')
+GOLDEN_FILE = 'reference_checks.pt'
+GRAD_SAMPLES = 32           # gradient entries stored per parameter tensor, with its L2 norm and GRAD_PROJECTIONS projections
+GRAD_PROJECTIONS = 4
 
 
 def _params(normalize_before, activation):
@@ -33,89 +31,65 @@ def _params(normalize_before, activation):
             'ctc_weight': 0.0, 'smoothing': 0.1}
 
 
-@pytest.mark.parametrize('normalize_before,activation', [(False, 'glu'), (True, 'relu')])
-def test_port_equals_live_reference(normalize_before, activation):
-    from otrans.model import End2EndModel
-    from otrans.recognize.speech2text import SpeechToTextRecognizer
-    params = _params(normalize_before, activation)
-    torch.manual_seed(4321)
-    ref = End2EndModel['speech2text'](params).eval()
-    with torch.no_grad():
-        ref.decoder.embedding.weight.mul_(0.15)
-        ref.decoder.output_layer.bias[1] = 1.5          # hypotheses end at different steps
-    sd = {k: v.detach().clone().float() for k, v in ref.state_dict().items() if k.split('.')[0] in ('frontend', 'encoder', 'decoder')}
-    g = torch.Generator().manual_seed(5)
-    B, T, beam, max_len = 3, 64, 3, 9
-    lens = torch.tensor([64, 50, 37])
+def grad_projections(flat, i):
+    """Seeded Gaussian projections of the flattened gradient of the i-th parameter: a deviation in any of its entries moves
+    them to first order, so together with the sampled entries and the norm they stand in for the full tensor."""
+    return torch.randn(GRAD_PROJECTIONS, flat.numel(), generator=torch.Generator().manual_seed(i)) @ flat
+
+
+def _batch(lens, T, g):
+    lens = torch.tensor(lens)
     mask = torch.arange(T)[None] < lens[:, None]
-    x = torch.randn(B, T, 20, generator=g) * mask.unsqueeze(2)
-    with torch.no_grad():
-        # encoder states: reference modules vs the port
-        fx, fm = ref.frontend(x, mask)
-        mem_ref, mm_ref, _ = ref.encoder(fx, fm)
-        mem, mm = om.encode(x, mask, sd, params)
-        assert torch.equal(mm, mm_ref)
-        torch.testing.assert_close(mem[mm], mem_ref[mm_ref], rtol=1e-4, atol=2e-5)
-        # the whole recognize(): ids bit-exact, scores to fp32 tolerance
-        rec = SpeechToTextRecognizer(ref, beam_width=beam, nbest=beam, max_len=max_len, idx2unit={i: str(i) for i in range(40)},
-                                     penalty=0.6, lamda=5, ngpu=0)
-        hyps, scores_ref = rec.recognize(x, mask)
-        nb, ns, _, _ = obs.recognize(x, mask, sd, params, beam=beam, nbest=beam, max_len=max_len, penalty=0.6, lamda=5)
-    for b in range(B):
-        for r in range(beam):
-            port = [int(t) for t in nb[b, r].tolist()]
-            port = port[:port.index(1)] if 1 in port else port
-            want = [int(t) for t in hyps[b][r].split()] if hyps[b][r] else []
-            assert port == want, (b, r, port, want)
-    torch.testing.assert_close(ns, scores_ref.float(), rtol=1e-4, atol=1e-4)
+    return torch.randn(len(lens), T, 20, generator=g) * mask.unsqueeze(2), mask
 
 
-@pytest.mark.parametrize('normalize_before,activation', [(False, 'glu'), (True, 'glu'), (False, 'relu'), (True, 'relu')])
-def test_port_gradients_equal_live_reference_autograd(normalize_before, activation):
-    """model.train(); loss, _ = model(inputs, targets); loss.backward() through the REFERENCE's own modules (trainer.py:206-217)
-    vs oracle/train_step.loss_and_grads: the loss and every parameter gradient -- in particular for the pre-norm and ReLU
-    stacks whose hand-written CUDA backward is tested against this port (tests/test_gpu_train.py)."""
-    from otrans.model import End2EndModel
-    from oracle import train_step as ot
-    params = _params(normalize_before, activation)
-    torch.manual_seed(99)
-    ref = End2EndModel['speech2text'](params)
-    ref.train()
+def random_weights(shapes, seed, eos_bias=None):
+    """Seeded weights for the state_dict layout `shapes` [(key, shape)]: linear / conv weights with the spread of nn.Linear's
+    default init, LayerNorm / BatchNorm parameters and running statistics away from their identity values, the shared
+    embedding scaled down.  `eos_bias` raises the output bias of <S/E> (id 1) so that hypotheses end at different steps."""
+    g = torch.Generator().manual_seed(seed)
+    sd = {}
+    for k, shape in shapes:
+        if k == 'decoder.output_layer.weight':         # share_embedding=True
+            sd[k] = sd['decoder.embedding.weight']
+        elif k.endswith('num_batches_tracked'):
+            sd[k] = torch.tensor(0)
+        elif k.endswith('running_mean'):
+            sd[k] = 0.3 * torch.randn(shape, generator=g)
+        elif k.endswith('running_var'):
+            sd[k] = 1.0 + 0.5 * torch.rand(shape, generator=g)
+        elif 'norm' in k:
+            sd[k] = (1.0 if k.endswith('weight') else 0.0) + 0.2 * torch.randn(shape, generator=g)
+        elif k == 'decoder.embedding.weight':
+            sd[k] = 0.15 * torch.randn(shape, generator=g)
+        elif k.endswith('.bias'):
+            sd[k] = 0.1 * torch.randn(shape, generator=g)
+        else:
+            sd[k] = torch.randn(shape, generator=g) / math.sqrt(3 * math.prod(shape[1:]))
+    if eos_bias is not None:
+        sd['decoder.output_layer.bias'][1] = eos_bias
+    return sd
+
+
+# Each case: (params, weight seed, <S/E> bias, inputs, search settings); make_reference_checks.py records the reference on them.
+def recognize_case(normalize_before, activation):
+    x, mask = _batch([64, 50, 37], 64, torch.Generator().manual_seed(5))
+    return _params(normalize_before, activation), 4321, 1.5, (x, mask), dict(beam=3, nbest=3, max_len=9, penalty=0.6, lamda=5)
+
+
+def gradient_case(normalize_before, activation):
     g = torch.Generator().manual_seed(7)
-    with torch.no_grad():
-        for n, p in ref.named_parameters():
-            if 'norm' in n:
-                p.add_(0.2 * torch.randn(p.shape, generator=g))
-            elif n.endswith('.bias'):
-                p.add_(0.05 * torch.randn(p.shape, generator=g))
-        ref.decoder.embedding.weight.mul_(0.12)
-    sd = {k: v.detach().clone().float() for k, v in ref.state_dict().items() if k.split('.')[0] in ('frontend', 'encoder', 'decoder')}
-    B, T, L = 3, 70, 8
-    lens = torch.tensor([70, 55, 41])
-    mask = torch.arange(T)[None] < lens[:, None]
-    x = torch.randn(B, T, 20, generator=g) * mask.unsqueeze(2)
+    x, mask = _batch([70, 55, 41], 70, g)
+    B, L = 3, 8
     tgt = torch.randint(3, 40, (B, L), generator=g)
     tgt[:, 0] = 1
     tgt[0, L - 2:] = torch.tensor([1, 0])
     tgt[1, L - 1] = 1
     tgt[2, 4:] = torch.tensor([1, 0, 0, 0])
-    loss_ref, _ = ref({'inputs': x, 'mask': mask}, {'targets': tgt, 'targets_length': None})
-    loss_ref.backward()
-    g_ref = {n: p.grad.clone() for n, p in ref.named_parameters() if p.grad is not None}
-    loss, grads = ot.loss_and_grads(x, mask, tgt, sd, params)
-    torch.testing.assert_close(loss, loss_ref.detach(), rtol=1e-5, atol=1e-5)
-    assert set(grads) == set(g_ref), set(grads) ^ set(g_ref)
-    for n in grads:
-        torch.testing.assert_close(grads[n], g_ref[n], rtol=2e-4, atol=2e-6, msg=lambda m, n=n: f'{n}: {m}')
+    return _params(normalize_before, activation), 99, None, (x, mask, tgt), None
 
 
-@pytest.mark.parametrize('kind', ['conformer', 'relpos_transformer'])
-def test_port_encoder_states_equal_live_reference_for_relpos_encoders(kind):
-    """Conformer (macaron FFN, rel-pos attention without output projection, conv module with BatchNorm running statistics,
-    only post_ffn_norm applied: SURVEY.md 8a quirks) and the rel-pos Transformer encoder: valid-frame states of the port vs
-    the live reference modules, recognize() ids bit-exact."""
-    from otrans.model import End2EndModel
-    from otrans.recognize.speech2text import SpeechToTextRecognizer
+def relpos_encoder_case(kind):
     params = _params(False, 'glu')
     if kind == 'conformer':
         params['encoder_type'] = 'conformer'
@@ -124,34 +98,93 @@ def test_port_encoder_states_equal_live_reference_for_relpos_encoders(kind):
                                  conv_bias=True, activation='glu', positional_encoding=True, relative_positional=True)
     else:
         params['encoder']['relative_positional'] = True
-    torch.manual_seed(77)
-    ref = End2EndModel['speech2text'](params).eval()
-    g = torch.Generator().manual_seed(11)
+    x, mask = _batch([72, 60, 33], 72, torch.Generator().manual_seed(11))
+    return params, 77, 1.5, (x, mask), dict(beam=3, nbest=1, max_len=7, penalty=0.6, lamda=5)
+
+
+RECOGNIZE = [(False, 'glu'), (True, 'relu')]
+GRADIENTS = [(False, 'glu'), (True, 'glu'), (False, 'relu'), (True, 'relu')]
+ENCODERS = ['conformer', 'relpos_transformer']
+
+
+def _name(family, *args):
+    return family + '/' + '-'.join(str(a) for a in args)
+
+
+def cases():
+    """(golden key, 'recognize' | 'gradients', case) of every test below."""
+    return ([(_name('recognize', *a), 'recognize', recognize_case(*a)) for a in RECOGNIZE]
+            + [(_name('gradients', *a), 'gradients', gradient_case(*a)) for a in GRADIENTS]
+            + [(_name('encoder', k), 'recognize', relpos_encoder_case(k)) for k in ENCODERS])
+
+
+@pytest.fixture(scope='module')
+def reference(golden_dir):
+    return torch.load(os.path.join(golden_dir, GOLDEN_FILE), weights_only=False)
+
+
+def _setup(reference, name, case):
+    params, seed, eos_bias, inputs, search = case
+    ref = reference[name]
+    return ref, params, random_weights(ref['shapes'], seed, eos_bias), inputs, search
+
+
+def _check_encoder(ref, x, mask, sd, params):
+    mem, mm = om.encode(x, mask, sd, params)
+    assert torch.equal(mm, ref['memory_mask'])
+    torch.testing.assert_close(mem[mm], ref['memory'], rtol=1e-4, atol=2e-5)
+
+
+def _port_hyps(nb, b, r):
+    port = [int(t) for t in nb[b, r].tolist()]
+    return port[:port.index(1)] if 1 in port else port
+
+
+@pytest.mark.parametrize('normalize_before,activation', RECOGNIZE)
+def test_port_equals_live_reference(reference, normalize_before, activation):
+    """Encoder states and the whole recognize(): ids bit-exact, scores to fp32 tolerance."""
+    ref, params, sd, (x, mask), s = _setup(reference, _name('recognize', normalize_before, activation),
+                                           recognize_case(normalize_before, activation))
     with torch.no_grad():
-        for n, buf in ref.named_buffers():
-            if n.endswith('running_mean'):
-                buf.add_(0.3 * torch.randn(buf.shape, generator=g))
-            if n.endswith('running_var'):
-                buf.mul_(1.0 + 0.5 * torch.rand(buf.shape, generator=g))
-        ref.decoder.embedding.weight.mul_(0.15)
-        ref.decoder.output_layer.bias[1] = 1.5
-    sd = {k: v.detach().clone().float() for k, v in ref.state_dict().items() if k.split('.')[0] in ('frontend', 'encoder', 'decoder')}
-    B, T, beam, max_len = 3, 72, 3, 7
-    lens = torch.tensor([72, 60, 33])
-    mask = torch.arange(T)[None] < lens[:, None]
-    x = torch.randn(B, T, 20, generator=g) * mask.unsqueeze(2)
+        _check_encoder(ref, x, mask, sd, params)
+        nb, ns, _, _ = obs.recognize(x, mask, sd, params, **s)
+    for b in range(x.shape[0]):
+        for r in range(s['beam']):
+            assert _port_hyps(nb, b, r) == ref['hyps'][b][r], (b, r)
+    torch.testing.assert_close(ns, ref['scores'], rtol=1e-4, atol=1e-4)
+
+
+@pytest.mark.parametrize('normalize_before,activation', GRADIENTS)
+def test_port_gradients_equal_live_reference_autograd(reference, normalize_before, activation):
+    """model.train(); loss, _ = model(inputs, targets); loss.backward() through the reference's own modules (trainer.py:206-217)
+    vs oracle/train_step.loss_and_grads: the loss, and for every parameter gradient its L2 norm and a seeded sample of its
+    entries -- in particular for the pre-norm and ReLU stacks whose hand-written CUDA backward is tested against this port
+    (tests/test_gpu_train.py)."""
+    from oracle import train_step as ot
+    ref, params, sd, (x, mask, tgt), _ = _setup(reference, _name('gradients', normalize_before, activation),
+                                                gradient_case(normalize_before, activation))
+    loss, grads = ot.loss_and_grads(x, mask, tgt, sd, params)
+    torch.testing.assert_close(loss, ref['loss'], rtol=1e-5, atol=1e-5)
+    assert set(grads) == set(ref['grad_names']), set(grads) ^ set(ref['grad_names'])
+    for i, n in enumerate(ref['grad_names']):
+        got = grads[n].reshape(-1)
+        torch.testing.assert_close(got[ref['grad_index'][i].long()], ref['grad_sample'][i], rtol=2e-4, atol=2e-6,
+                                   msg=lambda m, n=n: f'{n}: {m}')
+        torch.testing.assert_close(got.norm(), ref['grad_norm'][i], rtol=2e-4, atol=2e-6, msg=lambda m, n=n: f'{n} (L2 norm): {m}')
+        # entrywise errors within rtol / atol move a projection by about their L2 norm
+        tol = 4 * (2e-4 * float(ref['grad_norm'][i]) + 2e-6 * math.sqrt(got.numel()))
+        diff = float((grad_projections(got, i) - ref['grad_proj'][i]).abs().max())
+        assert diff <= tol, f'{n}: random projections differ by {diff:.3e} > {tol:.3e}'
+
+
+@pytest.mark.parametrize('kind', ENCODERS)
+def test_port_encoder_states_equal_live_reference_for_relpos_encoders(reference, kind):
+    """Conformer (macaron FFN, rel-pos attention without output projection, conv module with BatchNorm running statistics,
+    only post_ffn_norm applied: SURVEY.md 8a quirks) and the rel-pos Transformer encoder: valid-frame states of the port vs
+    the reference modules, recognize() ids bit-exact."""
+    ref, params, sd, (x, mask), s = _setup(reference, _name('encoder', kind), relpos_encoder_case(kind))
     with torch.no_grad():
-        fx, fm = ref.frontend(x, mask)
-        mem_ref, mm_ref, _ = ref.encoder(fx, fm)
-        mem, mm = om.encode(x, mask, sd, params)
-        assert torch.equal(mm, mm_ref)
-        torch.testing.assert_close(mem[mm], mem_ref[mm_ref], rtol=1e-4, atol=2e-5)
-        rec = SpeechToTextRecognizer(ref, beam_width=beam, nbest=1, max_len=max_len, idx2unit={i: str(i) for i in range(40)},
-                                     penalty=0.6, lamda=5, ngpu=0)
-        hyps, _ = rec.recognize(x, mask)
-        nb, _, _, _ = obs.recognize(x, mask, sd, params, beam=beam, nbest=1, max_len=max_len, penalty=0.6, lamda=5)
-    for b in range(B):
-        port = [int(t) for t in nb[b, 0].tolist()]
-        port = port[:port.index(1)] if 1 in port else port
-        want = [int(t) for t in hyps[b][0].split()] if hyps[b][0] else []
-        assert port == want, (b, port, want)
+        _check_encoder(ref, x, mask, sd, params)
+        nb, _, _, _ = obs.recognize(x, mask, sd, params, **s)
+    for b in range(x.shape[0]):
+        assert _port_hyps(nb, b, 0) == ref['hyps'][b][0], b
