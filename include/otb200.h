@@ -110,6 +110,13 @@ int otb_dropout_bwd(const void* dy, int lddy, void* out, int ldo, uint8_t* mask,
 int otb_attention(const void* q, int ldq, int q_rows, const void* k, int ldk, int k_rows, const void* v, int ldv,
                   void* out, int ldo, int B, int H, int Tq, int Tk, const int* kv_len, int causal, int q_col0,
                   int k_col0, int v_col0, const float* bd, int ldbd, const void* resid, int ldr, void* stream);
+/* otb_attention with the head width as an argument: head_dim 64 or 96 (d_model 384 with 4 heads, the Conformer
+ * recipe); head h starts at column *_col0 + head_dim*h and the scores are scaled by 1/sqrt(head_dim).  Any other
+ * head_dim returns a non-zero status (otb_last_error) without launching.  otb_attention is head_dim = 64. */
+int otb_attention_hd(const void* q, int ldq, int q_rows, const void* k, int ldk, int k_rows, const void* v, int ldv,
+                     void* out, int ldo, int B, int H, int head_dim, int Tq, int Tk, const int* kv_len, int causal,
+                     int q_col0, int k_col0, int v_col0, const float* bd, int ldbd, const void* resid, int ldr,
+                     void* stream);
 
 /* ConformerConvolutionModule middle (module/conformer.py:48-52): depthwise Conv1d(k, pad (k-1)/2) over time +
  * eval-mode BatchNorm1d + swish.  x, out bf16 [B*T, d]; w f32 [k, d] and b f32 [d] carry the BatchNorm affine
@@ -143,6 +150,10 @@ int otb_log_softmax(const float* x, int ldx, float* out, int ldo, int rows, int 
  * [Lmax,N,d]; anc i32 [2,N,Lmax]; *step_ptr = 0-based position; out bf16 [N,d]. */
 int otb_decode_self_attn(const void* qkv, void* kc, void* vc, const int* anc, const int* step_ptr, void* out, int N,
                          int H, int Lmax, void* stream);
+/* otb_decode_self_attn with the head width as an argument (64 or 96; d = H * head_dim).  otb_decode_self_attn is
+ * head_dim = 64. */
+int otb_decode_self_attn_hd(const void* qkv, void* kc, void* vc, const int* anc, const int* step_ptr, void* out, int N,
+                            int H, int head_dim, int Lmax, void* stream);
 
 /* LabelSmoothingLoss.forward (module/loss.py:21-48) fused: per-token KL(smoothed one-hot || softmax), PAD rows 0,
  * mean over non-PAD tokens.  logits f32 [rows, ldl]; targets i64 [rows]; tok_loss f32 [rows]; loss f32 [1];
@@ -231,7 +242,12 @@ int otb_attention_lse(const void* q, int ldq, int q_rows, const void* k, int ldk
                       void* out, int ldo, int B, int H, int Tq, int Tk, const int* kv_len, int causal, int q_col0,
                       int k_col0, int v_col0, const float* bd, int ldbd, const void* resid, int ldr, float* lse,
                       void* stream);
-/* Backward of otb_attention (no bd / resid): dq, dk, dv written at column offsets d*_col0 + 64*h of their matrices
+/* otb_attention_lse with the head width as an argument (64 or 96, as otb_attention_hd). */
+int otb_attention_lse_hd(const void* q, int ldq, int q_rows, const void* k, int ldk, int k_rows, const void* v, int ldv,
+                         void* out, int ldo, int B, int H, int head_dim, int Tq, int Tk, const int* kv_len, int causal,
+                         int q_col0, int k_col0, int v_col0, const float* bd, int ldbd, const void* resid, int ldr, float* lse,
+                         void* stream);
+/* Backward of otb_attention, head_dim = 64 only (no bd / resid): dq, dk, dv written at column offsets d*_col0 + 64*h of their matrices
  * (e.g. the three thirds of one [M,3d] dqkv buffer).  dsum f32 [B,H,Tq] is scratch.  tcgen05, scores recomputed. */
 int otb_attention_bwd(const void* q, int ldq, int q_rows, const void* k, int ldk, int k_rows, const void* v, int ldv,
                       const void* out, int ldo, const void* dout, int lddo, const float* lse, float* dsum, void* dq,

@@ -62,6 +62,7 @@ _SIGS = {
     'otb_embed_posenc': (c_int, [_P, c_int, _P, _P, _P, c_int, c_int, c_int, _P, c_int, _P]),
     'otb_log_softmax': (c_int, [_P, c_int, _P, c_int, c_int, c_int, _P]),
     'otb_decode_self_attn': (c_int, [_P, _P, _P, _P, _P, _P, c_int, c_int, c_int, _P]),
+    'otb_decode_self_attn_hd': (c_int, [_P, _P, _P, _P, _P, _P, c_int, c_int, c_int, c_int, _P]),
     'otb_ls_ce': (c_int, [_P, c_int, _P, c_int, c_int, c_float, c_int, _P, _P, _P, _P, c_int, _P]),
     'otb_beam_init': (c_int, [POINTER(BeamStateC), _P]),
     'otb_beam_step': (c_int, [_P, c_int, c_int, _P, c_int, c_float, POINTER(BeamStateC), _P, _P, _P]),
@@ -71,6 +72,10 @@ _SIGS = {
     'otb_beam_finalize': (c_int, [POINTER(BeamStateC), c_float, c_float, c_int, _P, _P, _P]),
     'otb_attention_lse': (c_int, [_P, c_int, c_int, _P, c_int, c_int, _P, c_int, _P, c_int, c_int, c_int, c_int, c_int,
                                   _P, c_int, c_int, c_int, c_int, _P, c_int, _P, c_int, _P, _P]),
+    'otb_attention_hd': (c_int, [_P, c_int, c_int, _P, c_int, c_int, _P, c_int, _P, c_int, c_int, c_int, c_int, c_int, c_int,
+                                 _P, c_int, c_int, c_int, c_int, _P, c_int, _P, c_int, _P]),
+    'otb_attention_lse_hd': (c_int, [_P, c_int, c_int, _P, c_int, c_int, _P, c_int, _P, c_int, c_int, c_int, c_int, c_int, c_int,
+                                     _P, c_int, c_int, c_int, c_int, _P, c_int, _P, c_int, _P, _P]),
     'otb_attention_bwd': (c_int, [_P, c_int, c_int, _P, c_int, c_int, _P, c_int, _P, c_int, _P, c_int, _P, _P, _P, c_int, c_int,
                                   _P, c_int, c_int, _P, c_int, c_int, c_int, c_int, c_int, c_int, _P, c_int, c_int, c_int, c_int, _P]),
     'otb_linear_wgrad': (c_int, [_P, c_int, _P, c_int, _P, c_int, c_int, c_int, c_int, c_int, _P]),

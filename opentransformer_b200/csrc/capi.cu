@@ -1,5 +1,6 @@
 // extern "C" boundary of libotb200.so (declared in include/otb200.h).  Argument checking, error
 // reporting (thread-local string, integer status, no aborts) and dispatch to the kernel launchers.
+#include <math.h>
 #include <stdio.h>
 #include <string.h>
 
@@ -177,27 +178,43 @@ int otb_dropout_bwd(const void* dy, int lddy, void* out, int ldo, uint8_t* mask,
 int otb_attention(const void* q, int ldq, int q_rows, const void* k, int ldk, int k_rows, const void* v, int ldv,
                   void* out, int ldo, int B, int H, int Tq, int Tk, const int* kv_len, int causal, int q_col0,
                   int k_col0, int v_col0, const float* bd, int ldbd, const void* resid, int ldr, void* stream) {
-    return otb_attention_lse(q, ldq, q_rows, k, ldk, k_rows, v, ldv, out, ldo, B, H, Tq, Tk, kv_len, causal, q_col0, k_col0,
-                             v_col0, bd, ldbd, resid, ldr, nullptr, stream);
+    return otb_attention_lse_hd(q, ldq, q_rows, k, ldk, k_rows, v, ldv, out, ldo, B, H, 64, Tq, Tk, kv_len, causal, q_col0,
+                                k_col0, v_col0, bd, ldbd, resid, ldr, nullptr, stream);
+}
+
+int otb_attention_hd(const void* q, int ldq, int q_rows, const void* k, int ldk, int k_rows, const void* v, int ldv,
+                     void* out, int ldo, int B, int H, int head_dim, int Tq, int Tk, const int* kv_len, int causal, int q_col0,
+                     int k_col0, int v_col0, const float* bd, int ldbd, const void* resid, int ldr, void* stream) {
+    return otb_attention_lse_hd(q, ldq, q_rows, k, ldk, k_rows, v, ldv, out, ldo, B, H, head_dim, Tq, Tk, kv_len, causal, q_col0,
+                                k_col0, v_col0, bd, ldbd, resid, ldr, nullptr, stream);
 }
 
 int otb_attention_lse(const void* q, int ldq, int q_rows, const void* k, int ldk, int k_rows, const void* v, int ldv,
                       void* out, int ldo, int B, int H, int Tq, int Tk, const int* kv_len, int causal, int q_col0,
                       int k_col0, int v_col0, const float* bd, int ldbd, const void* resid, int ldr, float* lse,
                       void* stream) {
+    return otb_attention_lse_hd(q, ldq, q_rows, k, ldk, k_rows, v, ldv, out, ldo, B, H, 64, Tq, Tk, kv_len, causal, q_col0,
+                                k_col0, v_col0, bd, ldbd, resid, ldr, lse, stream);
+}
+
+int otb_attention_lse_hd(const void* q, int ldq, int q_rows, const void* k, int ldk, int k_rows, const void* v, int ldv,
+                         void* out, int ldo, int B, int H, int head_dim, int Tq, int Tk, const int* kv_len, int causal,
+                         int q_col0, int k_col0, int v_col0, const float* bd, int ldbd, const void* resid, int ldr, float* lse,
+                         void* stream) {
+    if (head_dim != 64 && head_dim != 96) return fail("otb_attention", "head_dim must be 64 or 96");
     if (!q || !k || !v || !out) return fail("otb_attention", "null operand");
     if (q_col0 % 8 || k_col0 % 8 || v_col0 % 8 || ldo % 8) return fail("otb_attention", "column offsets / ldo must be multiples of 8");
     AttnParams p;
     p.B = B; p.H = H; p.Tq = Tq; p.Tk = Tk;
     p.kv_len = kv_len; p.causal = causal;
-    p.scale_log2 = 0.125f * 1.4426950408889634f;
+    p.scale_log2 = (head_dim == 64 ? 0.125f : 1.0f / sqrtf((float)head_dim)) * 1.4426950408889634f;
     p.out = reinterpret_cast<bf16*>(out); p.ldo = ldo;
     p.q_col0 = q_col0; p.k_col0 = k_col0; p.v_col0 = v_col0;
     p.bd = bd; p.ldbd = ldbd;
     p.resid = reinterpret_cast<const bf16*>(resid); p.ldr = ldr;
     p.lse = lse;
     if (resid && (ldr % 8)) return fail("otb_attention", "ldr must be a multiple of 8");
-    RET("otb_attention", attn_launch(ST(stream), q, ldq, q_rows, k, ldk, k_rows, v, ldv, p));
+    RET("otb_attention", attn_launch(ST(stream), q, ldq, q_rows, k, ldk, k_rows, v, ldv, p, head_dim));
 }
 
 int otb_layernorm(const void* x, int ldx, void* out, int ldo, int out_f32, const float* g1, const float* b1,
@@ -245,10 +262,16 @@ int otb_log_softmax(const float* x, int ldx, float* out, int ldo, int rows, int 
 
 int otb_decode_self_attn(const void* qkv, void* kc, void* vc, const int* anc, const int* step_ptr, void* out, int N,
                          int H, int Lmax, void* stream) {
+    return otb_decode_self_attn_hd(qkv, kc, vc, anc, step_ptr, out, N, H, 64, Lmax, stream);
+}
+
+int otb_decode_self_attn_hd(const void* qkv, void* kc, void* vc, const int* anc, const int* step_ptr, void* out, int N,
+                            int H, int head_dim, int Lmax, void* stream) {
+    if (head_dim != 64 && head_dim != 96) return fail("otb_decode_self_attn", "head_dim must be 64 or 96");
     if (!qkv || !kc || !vc || !anc || !step_ptr || !out) return fail("otb_decode_self_attn", "null operand");
     RET("otb_decode_self_attn",
         decode_self_attn_launch(ST(stream), reinterpret_cast<const bf16*>(qkv), reinterpret_cast<bf16*>(kc),
-                                reinterpret_cast<bf16*>(vc), anc, step_ptr, reinterpret_cast<bf16*>(out), N, H, Lmax));
+                                reinterpret_cast<bf16*>(vc), anc, step_ptr, reinterpret_cast<bf16*>(out), N, H, Lmax, head_dim));
 }
 
 int otb_ls_ce(const float* logits, int ldl, const int64_t* targets, int rows, int V, float smoothing, int pad_id,

@@ -619,16 +619,19 @@ static PFN_encodeTiled get_encode() {
 }
 
 const char* encode_tmap_2d(CUtensorMap* m, const void* base, uint64_t cols, uint64_t rows, uint64_t ld_elems,
-                           uint32_t box_cols, uint32_t box_rows) {
+                           uint32_t box_cols, uint32_t box_rows, int swizzle_bytes) {
     PFN_encodeTiled enc = get_encode();
     if (!enc) return "cuTensorMapEncodeTiled unavailable (no CUDA driver?)";
     if ((reinterpret_cast<uintptr_t>(base) & 15) || (ld_elems & 7)) return "TMA operand must be 16-byte aligned with ld % 8 == 0";
+    if (swizzle_bytes != 128 && swizzle_bytes != 64) return "encode_tmap_2d: swizzle must be 128 or 64 bytes";
+    if (box_cols * 2 > (uint32_t)swizzle_bytes) return "encode_tmap_2d: box row wider than the swizzle span";
     cuuint64_t dims[2] = {cols, rows};
     cuuint64_t strides[1] = {ld_elems * 2};
     cuuint32_t box[2] = {box_cols, box_rows};
     cuuint32_t estr[2] = {1, 1};
     CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                     CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
+                     CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     return r == CUDA_SUCCESS ? nullptr : "cuTensorMapEncodeTiled(2d) failed";
 }

@@ -385,50 +385,63 @@ const char* log_softmax_launch(cudaStream_t st, const float* x, int ldx, float* 
 // Decode-time self-attention with a per-hypothesis KV cache (the `cache` the reference stubbed out,
 // decoder/transformer.py:92-126,188-203).  One query (the newest token) per hypothesis; the prefix
 // K/V of hypothesis n at position s' < step live in slot anc[n][s'] of step s' (beam reordering
-// moves 4-byte ancestry entries, never K/V rows).  Warp = (hypothesis, head), d_k = 64, lane owns
-// two dims.  Also appends the current K/V to the cache.
+// moves 4-byte ancestry entries, never K/V rows).  Warp = (hypothesis, head), d_k = HD in {64, 96};
+// lane owns the bf16 pairs lane and lane + 32 (the latter only at HD = 96, lanes 0..15).
+// Also appends the current K/V to the cache.
 //   qkv   bf16 [N, 3d] (Q | K | V of the current token, attention.py:73 split order)
 //   kc,vc bf16 [Lmax, N, d]
 //   anc   int32 [2, N, Lmax]  (ping-pong, buffer (step & 1) is current)
 // ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128, 6) decode_self_attn_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ kc,
+template <int HD>
+__global__ void __launch_bounds__(128, HD == 64 ? 6 : 4) decode_self_attn_kernel(const bf16* __restrict__ qkv, bf16* __restrict__ kc,
                                                                bf16* __restrict__ vc, const int* __restrict__ anc,
                                                                const int* __restrict__ step_ptr, bf16* __restrict__ out,
                                                                int N, int H, int Lmax, float scale, int keys_pad) {
     PDL_TRIGGER();
     PDL_WAIT();
     // Lanes run over KEYS: each lane owns up to KPL cached positions, resolves their slots through the
-    // ancestry table and pulls the whole 128-byte K and V rows with 16-byte loads -- all loads of a lane are
+    // ancestry table and pulls the whole K and V rows (HD * 2 bytes) with 16-byte loads -- all loads of a lane are
     // independent, so the kernel costs ~3 dependent memory round trips (anc -> K/V -> out) instead of a
     // serial walk over the prefix.  V rows go through smem so that the P.V reduction is a column sum.
     constexpr int KPL = 4;               // keys per lane -> up to 128 cached positions
-    extern __shared__ uint4 sv_raw[];    // [warps][128 keys][8 x 16 B]  V rows (bf16)
+    constexpr int NC = HD / 8;           // 16-byte chunks per K/V row
+    constexpr int NP = HD / 2;           // bf16 pairs per row
+    // staged V row pitch in chunks: HD = 64 rotates the 8 chunks of row s by s; HD = 96 pads the 12 chunks to 13
+    // (an odd pitch spreads the 8 rows of a store phase over all 8 bank groups)
+    constexpr int PITCH = HD == 64 ? 8 : NC + 1;
+    extern __shared__ uint4 sv_raw[];    // [warps][keys_pad][PITCH x 16 B]  V rows (bf16)
     const int n = blockIdx.x;
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     const int nw = blockDim.x >> 5;
-    const int d = H * 64;
+    const int d = H * HD;
     const int step = *step_ptr;
     const int nkeys = step + 1;
     const int* an = anc + ((size_t)(step & 1) * N + n) * Lmax;
-    uint4* sv = sv_raw + (size_t)wib * keys_pad * 8;    // [keys_pad][8 x 16 B] per warp
-    // q lives in shared memory (every lane needs all 64 dims: 64 registers per thread otherwise, which capped the kernel
+    uint4* sv = sv_raw + (size_t)wib * keys_pad * PITCH;    // [keys_pad][PITCH x 16 B] per warp
+    // q lives in shared memory (every lane needs all HD dims: HD registers per thread otherwise, which capped the kernel
     // at 3 resident CTAs per SM -- the SM-time of this latency-bound kernel is what concurrent batches compete for)
-    float* sq = reinterpret_cast<float*>(sv_raw + (size_t)(blockDim.x >> 5) * keys_pad * 8) + wib * 64;
+    float* sq = reinterpret_cast<float*>(sv_raw + (size_t)(blockDim.x >> 5) * keys_pad * PITCH) + wib * HD;
+    auto v_word = [&](int s, int w) {    // 4-byte word w (dims 2w, 2w+1) of staged V row s
+        const uint32_t* svw = reinterpret_cast<const uint32_t*>(sv);
+        if constexpr (HD == 64) return svw[(s * 8 + (((w >> 2) + s) & 7)) * 4 + (w & 3)];   // chunks were rotated by s
+        else return svw[s * PITCH * 4 + w];
+    };
     for (int h = wib; h < H; h += nw) {
-        const bf16* base = qkv + (size_t)n * 3 * d + h * 64;
-        // append the newest K/V to the cache (lane owns dims 2*lane, 2*lane+1)
-        const uint32_t kcur = *reinterpret_cast<const uint32_t*>(base + d + 2 * lane);
-        const uint32_t vcur = *reinterpret_cast<const uint32_t*>(base + 2 * d + 2 * lane);
-        const size_t cur_off = ((size_t)step * N + n) * d + h * 64 + 2 * lane;
-        *reinterpret_cast<uint32_t*>(kc + cur_off) = kcur;
-        *reinterpret_cast<uint32_t*>(vc + cur_off) = vcur;
-        {
-            const float2 qq = unpack_bf16(*reinterpret_cast<const uint32_t*>(base + 2 * lane));
-            __syncwarp();
-            sq[2 * lane] = qq.x;
-            sq[2 * lane + 1] = qq.y;
-            __syncwarp();
+        const bf16* base = qkv + (size_t)n * 3 * d + h * HD;
+        // append the newest K/V to the cache
+        __syncwarp();
+#pragma unroll
+        for (int w = lane; w < NP; w += 32) {
+            const uint32_t kcur = *reinterpret_cast<const uint32_t*>(base + d + 2 * w);
+            const uint32_t vcur = *reinterpret_cast<const uint32_t*>(base + 2 * d + 2 * w);
+            const size_t cur_off = ((size_t)step * N + n) * d + h * HD + 2 * w;
+            *reinterpret_cast<uint32_t*>(kc + cur_off) = kcur;
+            *reinterpret_cast<uint32_t*>(vc + cur_off) = vcur;
+            const float2 qq = unpack_bf16(*reinterpret_cast<const uint32_t*>(base + 2 * w));
+            sq[2 * w] = qq.x;
+            sq[2 * w + 1] = qq.y;
         }
+        __syncwarp();
         int slot[KPL];
 #pragma unroll
         for (int j = 0; j < KPL; ++j) {
@@ -442,16 +455,16 @@ __global__ void __launch_bounds__(128, 6) decode_self_attn_kernel(const bf16* __
             const int s = lane + 32 * j;
             sc[j] = -INFINITY;
             if (s < nkeys) {   // warp-divergent only in the last group
-                const bf16* krow = (s == step) ? base + d : kc + ((size_t)s * N + slot[j]) * d + h * 64;
-                const bf16* vrow = (s == step) ? base + 2 * d : vc + ((size_t)s * N + slot[j]) * d + h * 64;
-                uint4 ku[8], vu[8];
+                const bf16* krow = (s == step) ? base + d : kc + ((size_t)s * N + slot[j]) * d + h * HD;
+                const bf16* vrow = (s == step) ? base + 2 * d : vc + ((size_t)s * N + slot[j]) * d + h * HD;
+                uint4 ku[NC], vu[NC];
 #pragma unroll
-                for (int i = 0; i < 8; ++i) ku[i] = *reinterpret_cast<const uint4*>(krow + 8 * i);
+                for (int i = 0; i < NC; ++i) ku[i] = *reinterpret_cast<const uint4*>(krow + 8 * i);
 #pragma unroll
-                for (int i = 0; i < 8; ++i) vu[i] = *reinterpret_cast<const uint4*>(vrow + 8 * i);
+                for (int i = 0; i < NC; ++i) vu[i] = *reinterpret_cast<const uint4*>(vrow + 8 * i);
                 float dot = 0.f;
 #pragma unroll
-                for (int i = 0; i < 8; ++i) {
+                for (int i = 0; i < NC; ++i) {
                     const float2 a = unpack_bf16(ku[i].x), b = unpack_bf16(ku[i].y), c = unpack_bf16(ku[i].z),
                                  e = unpack_bf16(ku[i].w);
                     const float4 q0 = *reinterpret_cast<const float4*>(sq + 8 * i);      // broadcast reads
@@ -461,7 +474,10 @@ __global__ void __launch_bounds__(128, 6) decode_self_attn_kernel(const bf16* __
                 sc[j] = dot * scale;
                 mx = fmaxf(mx, sc[j]);
 #pragma unroll
-                for (int i = 0; i < 8; ++i) sv[s * 8 + ((i + s) & 7)] = vu[i];   // rotate chunks: conflict-free rows
+                for (int i = 0; i < NC; ++i) {
+                    if constexpr (HD == 64) sv[s * 8 + ((i + s) & 7)] = vu[i];   // rotate chunks: conflict-free rows
+                    else sv[s * PITCH + i] = vu[i];
+                }
             }
         }
         mx = warp_max(mx);
@@ -473,9 +489,12 @@ __global__ void __launch_bounds__(128, 6) decode_self_attn_kernel(const bf16* __
         }
         l = warp_sum(l);
         __syncwarp();
-        // P.V as a column sum over the staged V rows: lane owns output dims 2*lane, 2*lane+1
-        const uint32_t* svw = reinterpret_cast<const uint32_t*>(sv);
-        float ax = 0.f, ay = 0.f;
+        // P.V as a column sum over the staged V rows: lane owns the bf16 pairs lane (+ lane + 32)
+        constexpr int NW = (NP + 31) / 32;
+        const bool second = NW > 1 && lane + 32 < NP;
+        float ax[NW], ay[NW];
+#pragma unroll
+        for (int u = 0; u < NW; ++u) ax[u] = ay[u] = 0.f;
 #pragma unroll
         for (int j = 0; j < KPL; ++j) {
             const int cnt = min(32, nkeys - 32 * j);
@@ -484,36 +503,56 @@ __global__ void __launch_bounds__(128, 6) decode_self_attn_kernel(const bf16* __
             for (int t = 0; t < cnt; ++t) {
                 const int s = t + 32 * j;
                 const float pw = __shfl_sync(0xffffffffu, sc[j], t);
-                // dims 2*lane.. live in 16-byte chunk (lane >> 2), word (lane & 3); chunks were rotated by s
-                const uint32_t vv = svw[(s * 8 + (((lane >> 2) + s) & 7)) * 4 + (lane & 3)];
-                const float2 vf = unpack_bf16(vv);
-                ax = fmaf(pw, vf.x, ax);
-                ay = fmaf(pw, vf.y, ay);
+                const float2 vf = unpack_bf16(v_word(s, lane));
+                ax[0] = fmaf(pw, vf.x, ax[0]);
+                ay[0] = fmaf(pw, vf.y, ay[0]);
+                if constexpr (NW > 1) {
+                    if (second) {
+                        const float2 vg = unpack_bf16(v_word(s, lane + 32));
+                        ax[NW - 1] = fmaf(pw, vg.x, ax[NW - 1]);
+                        ay[NW - 1] = fmaf(pw, vg.y, ay[NW - 1]);
+                    }
+                }
             }
         }
         const float inv = 1.0f / l;
-        *reinterpret_cast<uint32_t*>(out + (size_t)n * d + h * 64 + 2 * lane) = pack_bf16(ax * inv, ay * inv);
+        bf16* orow = out + (size_t)n * d + h * HD;
+        *reinterpret_cast<uint32_t*>(orow + 2 * lane) = pack_bf16(ax[0] * inv, ay[0] * inv);
+        if constexpr (NW > 1) {
+            if (second) *reinterpret_cast<uint32_t*>(orow + 2 * (lane + 32)) = pack_bf16(ax[NW - 1] * inv, ay[NW - 1] * inv);
+        }
         __syncwarp();
     }
 }
 
-const char* decode_self_attn_launch(cudaStream_t st, const bf16* qkv, bf16* kc, bf16* vc, const int* anc,
-                                    const int* step_ptr, bf16* out, int N, int H, int Lmax) {
-    if (Lmax > 128) return "decode_self_attn: at most 128 cached positions (max_len <= 128)";
+template <int HD>
+static const char* decode_self_attn_launch_hd(cudaStream_t st, const bf16* qkv, bf16* kc, bf16* vc, const int* anc,
+                                              const int* step_ptr, bf16* out, int N, int H, int Lmax) {
     const int warps = H < 4 ? H : 4;
     // V staging sized by the longest prefix this search can reach (not the 128-key maximum): at max_len 60 this halves the
     // shared memory per CTA and doubles the resident CTAs of this latency-bound kernel (less SM-time per decode step)
+    constexpr int PITCH = HD == 64 ? 8 : HD / 8 + 1;
+    constexpr int MAX_SMEM = 4 * 128 * PITCH * 16 + 4 * HD * (int)sizeof(float);
     const int keys_pad = (Lmax + 31) / 32 * 32;
-    const size_t smem = (size_t)warps * keys_pad * 128 + (size_t)warps * 64 * sizeof(float);   // V rows | q per warp
+    const size_t smem = (size_t)warps * keys_pad * PITCH * 16 + (size_t)warps * HD * sizeof(float);   // V rows | q per warp
     static bool attr_set = false;
     if (!attr_set) {
-        if (cudaFuncSetAttribute(decode_self_attn_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 80 * 1024) != cudaSuccess)
+        if (cudaFuncSetAttribute(decode_self_attn_kernel<HD>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 MAX_SMEM > 80 * 1024 ? MAX_SMEM : 80 * 1024) != cudaSuccess)
             return "cudaFuncSetAttribute(decode_self_attn) failed";
         attr_set = true;
     }
-    cudaError_t e = launch_pdl(decode_self_attn_kernel, dim3(N), dim3(warps * 32), smem, st, qkv, kc, vc, anc, step_ptr, out, N, H, Lmax,
-                               0.125f, keys_pad);
+    cudaError_t e = launch_pdl(decode_self_attn_kernel<HD>, dim3(N), dim3(warps * 32), smem, st, qkv, kc, vc, anc, step_ptr, out, N,
+                               H, Lmax, HD == 64 ? 0.125f : 1.0f / sqrtf((float)HD), keys_pad);
     return e == cudaSuccess ? nullptr : cudaGetErrorString(e);
+}
+
+const char* decode_self_attn_launch(cudaStream_t st, const bf16* qkv, bf16* kc, bf16* vc, const int* anc,
+                                    const int* step_ptr, bf16* out, int N, int H, int Lmax, int head_dim) {
+    if (Lmax > 128) return "decode_self_attn: at most 128 cached positions (max_len <= 128)";
+    if (head_dim == 64) return decode_self_attn_launch_hd<64>(st, qkv, kc, vc, anc, step_ptr, out, N, H, Lmax);
+    if (head_dim == 96) return decode_self_attn_launch_hd<96>(st, qkv, kc, vc, anc, step_ptr, out, N, H, Lmax);
+    return "head_dim must be 64 or 96";
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -64,8 +64,9 @@ const char* gemm_wgrad_launch(cudaStream_t st, const void* dY, int lddy, const v
                               int Mact, int Nw, int Kw, int accumulate);
 
 // encode helpers (driver entry point fetched at runtime; libcuda is not a link-time dependency)
+// swizzle_bytes: 128 (box of <= 64 columns) or 64 (box of <= 32 columns)
 const char* encode_tmap_2d(CUtensorMap* m, const void* base, uint64_t cols, uint64_t rows, uint64_t ld_elems,
-                           uint32_t box_cols, uint32_t box_rows);
+                           uint32_t box_cols, uint32_t box_rows, int swizzle_bytes = 128);
 const char* encode_tmap_2d_f32(CUtensorMap* m, const void* base, uint64_t cols, uint64_t rows, uint64_t ld_elems,
                                uint32_t box_cols, uint32_t box_rows);
 const char* encode_tmap_conv5d(CUtensorMap* m, const void* base, int C, int F1h, int T1h_total, uint32_t boxF,
@@ -203,7 +204,7 @@ size_t decode_group_workspace_bytes(int N, int n_layers, int Lmax, int B, int be
 const char* decode_group_launch(cudaStream_t st, const MegaParams& p, void* workspace, size_t workspace_bytes);
 
 const char* attn_launch(cudaStream_t st, const void* q, int ldq, int q_rows, const void* k, int ldk, int k_rows,
-                        const void* v, int ldv, const AttnParams& p);
+                        const void* v, int ldv, const AttnParams& p, int head_dim);   // head_dim 64 or 96
 const char* conv1_launch(cudaStream_t st, const float* x, const float* w, const float* bias, bf16* out, int B, int T,
                          int F, int T1, int F1, int T1pad, int F1pad, int C1);
 const char* layernorm_launch(cudaStream_t st, const bf16* x, int ldx, void* out, int ldo, int out_f32, const float* g1,
@@ -218,7 +219,7 @@ const char* embed_posenc_launch(cudaStream_t st, const long long* tok, int tok_s
                                 int vocab);
 const char* log_softmax_launch(cudaStream_t st, const float* x, int ldx, float* out, int ldo, int rows, int V);
 const char* decode_self_attn_launch(cudaStream_t st, const bf16* qkv, bf16* kc, bf16* vc, const int* anc,
-                                    const int* step_ptr, bf16* out, int N, int H, int Lmax);
+                                    const int* step_ptr, bf16* out, int N, int H, int Lmax, int head_dim);
 const char* beam_init_launch(cudaStream_t stream, BeamState st);
 const char* beam_step_launch(cudaStream_t stream, const float* logp, int ldl, int V, const float* lm_logp, int ld_lm,
                              float lm_weight, BeamState st, long long* dbg_ktok, int* dbg_offs, const float* pre_val,

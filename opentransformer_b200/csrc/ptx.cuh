@@ -222,6 +222,12 @@ __device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t smem_addr, uint32_t
     return (uint64_t)((smem_addr >> 4) & 0x3FFF) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16) |
            ((uint64_t)((sbo_bytes >> 4) & 0x3FFF) << 32) | (1ull << 46) | (2ull << 61);
 }
+// The same for a tile of 32 bf16 (64 B) per row, 64-byte swizzle (layout type 4): 8-row groups are 512 B apart.
+// Used as K-major operand (k-steps at +32 B inside the row) and as MN-major B operand with N = 32 (one atom wide).
+__device__ __forceinline__ uint64_t umma_desc_sw64(uint32_t smem_addr) {
+    return (uint64_t)((smem_addr >> 4) & 0x3FFF) | ((uint64_t)1 << 16) | ((uint64_t)(512 >> 4) << 32) | (1ull << 46) |
+           (4ull << 61);
+}
 // Instruction descriptor for kind::f16, BF16 x BF16 -> FP32, M = 128:
 //   [4,6) D format (1 = F32) | [7,10) A format (1 = BF16) | [10,13) B format | [15] A major | [16] B major
 //   [17,23) N >> 3 | [24,29) M >> 4

@@ -24,6 +24,9 @@ class TransformerLanguageModel(nn.Module):
         self.vocab_size = params['vocab_size']
         self.num_blocks = params['num_blocks']
         self.d_model = params['d_model']
+        if self.d_model != params['n_heads'] * 64:
+            # the layers would run at d_k = 96 too, but that LM path has no parity test yet
+            raise NotImplementedError('TransformerLanguageModel: d_k = d_model / n_heads must be 64')
         self.embedding = nn.Embedding(self.vocab_size, self.d_model)
         self.pos_embedding = PositionalEncoding(self.d_model, 0.0)
         self.blocks = nn.ModuleList([

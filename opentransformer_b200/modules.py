@@ -67,6 +67,17 @@ def _ln(norm):
     return norm.weight.detach().float().contiguous(), norm.bias.detach().float().contiguous()
 
 
+HEAD_DIMS = (64, 96)   # head widths the sm_100a attention kernels are built for
+
+
+def head_dim_of(n_heads, d_model):
+    """d_model // n_heads when it is a head width the attention kernels support, else NotImplementedError."""
+    if n_heads < 1 or d_model % n_heads or d_model // n_heads not in HEAD_DIMS:
+        raise NotImplementedError(f'the sm_100a attention kernels support d_k = d_model / n_heads in {HEAD_DIMS}; '
+                                  f'got d_model {d_model}, n_heads {n_heads}')
+    return d_model // n_heads
+
+
 def _no_train(module):
     if module.training and torch.is_grad_enabled():
         raise NotImplementedError('module-level forward is the inference path: call under model.eval() / torch.no_grad(); '
@@ -183,8 +194,7 @@ class MultiHeadedSelfAttention(nn.Module):
         super().__init__()
         if share_qvk_proj:
             raise NotImplementedError('share_qvk_proj')
-        if d_model != n_heads * 64:
-            raise NotImplementedError('the sm_100a attention kernel is specialised for d_k = 64')
+        self.head_dim = head_dim_of(n_heads, d_model)
         self.qvk_proj = nn.Linear(d_model, d_model * 3)
         self.output_proj = nn.Linear(d_model, d_model)
 
@@ -196,8 +206,7 @@ class MultiHeadedCrossAttention(nn.Module):
         super().__init__()
         if share_vk_proj:
             raise NotImplementedError('share_vk_proj')
-        if d_model != n_heads * 64:
-            raise NotImplementedError('the sm_100a attention kernel is specialised for d_k = 64')
+        self.head_dim = head_dim_of(n_heads, d_model)
         self.q_proj = nn.Linear(d_model, d_model)
         self.vk_proj = nn.Linear(memory_dim, d_model * 2)
         self.output_proj = nn.Linear(d_model, d_model)
@@ -304,7 +313,7 @@ class TransformerEncoderLayer(nn.Module):
             return _ffn(x, pk['ffn'], x, None if self.normalize_before else pk['ln2'])
         qkv = ops.linear(x, pk['wqkv'], pk['bqkv'])
         ctx = ops.attention(qkv, qkv, qkv, B, H, T, T, kv_len=lengths, causal=causal, q_col0=0, k_col0=d,
-                            v_col0=2 * d)
+                            v_col0=2 * d, head_dim=self.slf_attn.head_dim)
         x = _proj_resid_ln(ctx, pk['wo'], pk['bo'], x, None if self.normalize_before else pk['ln1'])
         if self.normalize_before:
             x = ops.layernorm(x, *pk['ln2'])
@@ -385,8 +394,7 @@ class MultiHeadedSelfAttentionWithRelPos(nn.Module):
         super().__init__()
         if dropout_rate or skip_term_b or share_qvk_proj:
             raise NotImplementedError('rel-pos attention: dropout / skip_term_b / share_qvk_proj')
-        if d_model != n_heads * 64:
-            raise NotImplementedError('the sm_100a attention kernel is specialised for d_k = 64')
+        self.head_dim = head_dim_of(n_heads, d_model)
         self.nheads, self.d_model = n_heads, d_model
         self.qvk_proj = nn.Linear(d_model, d_model * 3)
         self.pos_proj = nn.Linear(d_model, d_model, bias=False)
@@ -406,15 +414,16 @@ class MultiHeadedSelfAttentionWithRelPos(nn.Module):
 
     def run(self, y, x_resid, pk, B, T, lengths, pos_bf16):
         """y = LN(x) bf16 [B*T,d]; returns x_resid + attention (no output projection)."""
-        d, H = self.d_model, self.nheads
+        d, H, dk = self.d_model, self.nheads, self.head_dim
         ext = ops.linear(y, pk['wext'], pk['bext'])                       # [M, 4d]
         pproj = ops.linear(pos_bf16, pk['wpos'])                          # [2T-1, d]  pos_proj(PE[-(T-1)..T-1])
         ld = (2 * T - 1 + 3) // 4 * 4
         bd = torch.empty(H, B * T, ld, dtype=torch.float32, device=y.device)
         for h in range(H):  # BD_full[h] = (q+v)_h P_h^T ; the attention kernel reads the j-i+T-1 diagonal band
-            ops.linear(ext[:, d + 64 * h: d + 64 * (h + 1)], pproj[:, 64 * h: 64 * (h + 1)], out=bd[h])
+            # K = dk column views: the GEMM's TMA maps are bounded by K, so a 64-column k-block past the head zero-fills
+            ops.linear(ext[:, d + dk * h: d + dk * (h + 1)], pproj[:, dk * h: dk * (h + 1)], out=bd[h])
         return ops.attention(ext, ext, ext, B, H, T, T, kv_len=lengths, q_col0=0, k_col0=2 * d, v_col0=3 * d,
-                             bd=bd, resid=x_resid)
+                             bd=bd, resid=x_resid, head_dim=dk)
 
 
 class ConformerConvolutionModule(nn.Module):
@@ -488,7 +497,8 @@ class ConformerEncoderBlock(nn.Module):
             return self.mha.run(y, x, pk['mha'], B, T, lengths, pos_bf16)
         d, H, m = x.shape[1], self.n_heads, pk['mha']
         qkv = ops.linear(y, m['wqkv'], m['bqkv'])
-        ctx = ops.attention(qkv, qkv, qkv, B, H, T, T, kv_len=lengths, q_col0=0, k_col0=d, v_col0=2 * d)
+        ctx = ops.attention(qkv, qkv, qkv, B, H, T, T, kv_len=lengths, q_col0=0, k_col0=d, v_col0=2 * d,
+                            head_dim=self.mha.head_dim)
         return ops.linear(ctx, m['wo'], m['bo'], EPI_RESID, resid=x)
 
     def _conv(self, x, pk, B, T, lengths):
@@ -659,6 +669,7 @@ class TransformerDecoder(nn.Module):
         self.normalize_before = normalize_before
         self.relative_positional = False
         self.d_model, self.n_heads, self.vocab_size = d_model, n_heads, vocab_size
+        self.head_dim = head_dim_of(n_heads, d_model)
         self.embedding = nn.Embedding(vocab_size, d_model)
         self.pos_emb = PositionalEncoding(d_model, pos_dropout)
         self.blocks = nn.ModuleList([
@@ -701,13 +712,13 @@ class TransformerDecoder(nn.Module):
             if nb:
                 x = ops.layernorm(x, *p['ln1'])
             qkv = ops.linear(x, p['wqkv'], p['bqkv'])
-            ctx = ops.attention(qkv, qkv, qkv, B, H, L, L, causal=True, q_col0=0, k_col0=d, v_col0=2 * d)
+            ctx = ops.attention(qkv, qkv, qkv, B, H, L, L, causal=True, q_col0=0, k_col0=d, v_col0=2 * d, head_dim=self.head_dim)
             x = _proj_resid_ln(ctx, p['wo'], p['bo'], x, None if nb else p['ln1'])
             if nb:
                 x = ops.layernorm(x, *p['ln2'])
             q = ops.linear(x, p['wq'], p['bq'])
             kv = ops.linear(memory_bf16, p['wkv'], p['bkv'])
-            ctx = ops.attention(q, kv, kv, B, H, L, T, kv_len=mem_len, k_col0=0, v_col0=d)
+            ctx = ops.attention(q, kv, kv, B, H, L, T, kv_len=mem_len, k_col0=0, v_col0=d, head_dim=self.head_dim)
             x = _proj_resid_ln(ctx, p['wo2'], p['bo2'], x, None if nb else p['ln2'])
             if nb:
                 x = ops.layernorm(x, *p['ln3'])
@@ -762,12 +773,13 @@ class TransformerDecoder(nn.Module):
             if nb:
                 x = ops.layernorm(x, *p['ln1'])
             qkv = ops.linear(x, p['wqkv'], p['bqkv'])
-            ctx = ops.decode_self_attn(qkv, c.kc[l], c.vc[l], c.anc, c.step_dev, N, H, c.Lmax)
+            ctx = ops.decode_self_attn(qkv, c.kc[l], c.vc[l], c.anc, c.step_dev, N, H, c.Lmax, head_dim=self.head_dim)
             x = _proj_resid_ln(ctx, p['wo'], p['bo'], x, None if nb else p['ln1'])
             if nb:
                 x = ops.layernorm(x, *p['ln2'])
             q = ops.linear(x, p['wq'], p['bq'])
-            ctx = ops.attention(q, c.kvx[l], c.kvx[l], c.batch, H, c.beam, c.T, kv_len=c.mem_len, k_col0=0, v_col0=d)
+            ctx = ops.attention(q, c.kvx[l], c.kvx[l], c.batch, H, c.beam, c.T, kv_len=c.mem_len, k_col0=0, v_col0=d,
+                                head_dim=self.head_dim)
             x = _proj_resid_ln(ctx, p['wo2'], p['bo2'], x, None if nb else p['ln2'])
             if nb:
                 x = ops.layernorm(x, *p['ln3'])

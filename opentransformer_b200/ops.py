@@ -177,19 +177,20 @@ def dropout_mask(M, N, p, seed, site):
 
 
 def attention(q, k, v, B, H, Tq, Tk, kv_len=None, causal=False, q_col0=0, k_col0=0, v_col0=0, out=None, bd=None,
-              resid=None):
-    """q/k/v: bf16 2-D matrices (may be the same [M,3d] buffer with different column offsets)."""
+              resid=None, head_dim=64):
+    """q/k/v: bf16 2-D matrices (may be the same [M,3d] buffer with different column offsets); head h reads columns
+    *_col0 + head_dim*h (head_dim 64 or 96)."""
     for t, n in ((q, 'q'), (k, 'k'), (v, 'v')):
         _need(t, BF16, n)
-    d = H * 64
+    d = H * head_dim
     if out is None:
         out = torch.empty(B * Tq, d, dtype=BF16, device=q.device)
     if kv_len is not None:
         _need(kv_len, torch.int32, 'kv_len')
-    check(_lib.lib().otb_attention(_p(q), q.stride(0), q.shape[0], _p(k), k.stride(0), k.shape[0], _p(v), v.stride(0),
-                                   _p(out), out.stride(0), B, H, Tq, Tk, _p(kv_len), 1 if causal else 0, q_col0,
-                                   k_col0, v_col0, _p(bd), bd.shape[-1] if bd is not None else 0, _p(resid),
-                                   resid.stride(0) if resid is not None else 0, _stream()),
+    check(_lib.lib().otb_attention_hd(_p(q), q.stride(0), q.shape[0], _p(k), k.stride(0), k.shape[0], _p(v), v.stride(0),
+                                      _p(out), out.stride(0), B, H, head_dim, Tq, Tk, _p(kv_len), 1 if causal else 0, q_col0,
+                                      k_col0, v_col0, _p(bd), bd.shape[-1] if bd is not None else 0, _p(resid),
+                                      resid.stride(0) if resid is not None else 0, _stream()),
           'otb_attention')
     _count()
     return out
@@ -301,11 +302,11 @@ def ls_cross_entropy(logits, targets, V, smoothing=0.1, pad_id=0, want_grad=Fals
     return loss[0], dl
 
 
-def decode_self_attn(qkv, kc, vc, anc, step_ptr, N, H, Lmax, out=None):
+def decode_self_attn(qkv, kc, vc, anc, step_ptr, N, H, Lmax, out=None, head_dim=64):
     if out is None:
-        out = torch.empty(N, H * 64, dtype=BF16, device=qkv.device)
-    check(_lib.lib().otb_decode_self_attn(_p(qkv), _p(kc), _p(vc), _p(anc), _p(step_ptr), _p(out), N, H, Lmax,
-                                          _stream()), 'otb_decode_self_attn')
+        out = torch.empty(N, H * head_dim, dtype=BF16, device=qkv.device)
+    check(_lib.lib().otb_decode_self_attn_hd(_p(qkv), _p(kc), _p(vc), _p(anc), _p(step_ptr), _p(out), N, H, head_dim, Lmax,
+                                             _stream()), 'otb_decode_self_attn')
     _count()
     return out
 
@@ -384,15 +385,16 @@ def decode_persistent(model_c, kvx, mem_len, kc, vc, state, B, T, max_steps, wor
 # ------------------------------------------------------------------------------------------------
 # training step: backward kernels (include/otb200.h "Training step")
 # ------------------------------------------------------------------------------------------------
-def attention_train(q, k, v, B, H, Tq, Tk, kv_len=None, causal=False, q_col0=0, k_col0=0, v_col0=0):
-    """otb_attention + the per-row log-sum-exp the backward needs -> (out bf16 [B*Tq, H*64], lse f32 [B,H,Tq])."""
+def attention_train(q, k, v, B, H, Tq, Tk, kv_len=None, causal=False, q_col0=0, k_col0=0, v_col0=0, head_dim=64):
+    """otb_attention + the per-row log-sum-exp the backward needs -> (out bf16 [B*Tq, H*head_dim], lse f32 [B,H,Tq]).
+    (attention_bwd is 64-wide only.)"""
     for t, n in ((q, 'q'), (k, 'k'), (v, 'v')):
         _need(t, BF16, n)
-    out = torch.empty(B * Tq, H * 64, dtype=BF16, device=q.device)
+    out = torch.empty(B * Tq, H * head_dim, dtype=BF16, device=q.device)
     lse = torch.empty(B, H, Tq, dtype=torch.float32, device=q.device)
-    check(_lib.lib().otb_attention_lse(_p(q), q.stride(0), q.shape[0], _p(k), k.stride(0), k.shape[0], _p(v), v.stride(0),
-                                       _p(out), out.stride(0), B, H, Tq, Tk, _p(kv_len), 1 if causal else 0, q_col0, k_col0,
-                                       v_col0, None, 0, None, 0, _p(lse), _stream()), 'otb_attention_lse')
+    check(_lib.lib().otb_attention_lse_hd(_p(q), q.stride(0), q.shape[0], _p(k), k.stride(0), k.shape[0], _p(v), v.stride(0),
+                                          _p(out), out.stride(0), B, H, head_dim, Tq, Tk, _p(kv_len), 1 if causal else 0, q_col0,
+                                          k_col0, v_col0, None, 0, None, 0, _p(lse), _stream()), 'otb_attention_lse')
     _count()
     return out, lse
 

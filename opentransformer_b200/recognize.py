@@ -176,7 +176,7 @@ class BeamDecoder:
             if nb:
                 x = ops.layernorm(x, *p['ln1'])
             qkv = ops.linear(x, p['wqkv'], p['bqkv'])
-            ctx = ops.decode_self_attn(qkv, self.kc[l], self.vc[l], st.anc, st.step_ptr, N, H, self.Lmax)
+            ctx = ops.decode_self_attn(qkv, self.kc[l], self.vc[l], st.anc, st.step_ptr, N, H, self.Lmax, head_dim=dec.head_dim)
             x = _proj_resid_ln(ctx, p['wo'], p['bo'], x, None if nb else p['ln1'])
             if nb:
                 x = ops.layernorm(x, *p['ln2'])
@@ -185,7 +185,7 @@ class BeamDecoder:
             # (a SIMT kernel specialised for <= 16 query rows was measured at 14.9 us against 10.0 us for this tcgen05 kernel
             # padded to 128 rows and was dropped: profiles/r1_bench_history.md)
             ctx = ops.attention(q, self.kvx[l], self.kvx[l], self.B, H, self.beam, self.T, kv_len=self.mem_len,
-                                k_col0=0, v_col0=d)
+                                k_col0=0, v_col0=d, head_dim=dec.head_dim)
             x = _proj_resid_ln(ctx, p['wo2'], p['bo2'], x, None if nb else p['ln2'])
             if nb:
                 x = ops.layernorm(x, *p['ln3'])

@@ -47,6 +47,11 @@ class TrainPack:
             raise NotImplementedError('training path: conv front end + Transformer encoder / decoder only (round 1)')
         if enc.relative_positional:
             raise NotImplementedError('training path: absolute positions only')
+        for blk in list(enc.blocks) + list(dec.blocks):
+            if blk.slf_attn.head_dim != 64:
+                # the attention backward kernel (otb_attention_bwd) is built for 64-wide heads only
+                raise NotImplementedError(f'training path: the attention backward supports d_k = 64 only, '
+                                          f'got d_k = {blk.slf_attn.head_dim}')
         if fe.front_end_layer_norm or enc.pos_emb.scale_learnable or dec.pos_emb.scale_learnable:
             raise NotImplementedError('training path: front_end_layer_norm / learnable positional scale')
         for blk in list(enc.blocks) + list(dec.blocks):
